@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- entities/s through propagate -> cull -> cluster (BASELINE.json's metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--scaling strong|weak]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--scaling strong|weak] [--dump-outputs DIR]
 
 A "step" is one frame of the hot path over the synthetic config-#3 scene: 1,000,110 hierarchy entities (3922 complete
 binary trees, depth 8, BFS order) + 256 point lights, 4 view frusta, 1920x1080, default ClusterConfig.  Every frame all
@@ -27,6 +27,8 @@ path) and the cameras rotate.
   parity        outside the timed regions the frame that follows each timed loop is checked bit for bit against the CPU
                 oracle (GlobalTransform bits, both change columns, ViewVisibility, sorted visible lists, cluster CSR, column
                 write-back) on every rank: `parity_checked`.
+  outputs       --dump-outputs DIR writes the results of the last step of the device-resident timed loop as .npy files
+                (dump_outputs); the inputs are seeded, so two builds run with the same arguments compute the same frame.
 """
 import argparse
 import ctypes
@@ -70,6 +72,7 @@ def parse_args():
     ap.add_argument("--no-parity", action="store_true", help="skip the oracle checks (they run outside the timed regions)")
     ap.add_argument("--no-secondary", action="store_true", help="N > 1: skip the other scaling mode's short measurement")
     ap.add_argument("--print-config", action="store_true", help="print the `config` object of this command line and exit")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step as DIR/<name>.npy (b200 arm)")
     return ap.parse_args()
 
 
@@ -225,6 +228,8 @@ def cpu_summary(times, n, threads, what, calibration=""):
 
 
 def run_reference(args):
+    if args.dump_outputs:
+        raise SystemExit("--dump-outputs writes the b200 arm's results; the reference arm has none to write")
     if int(os.environ.get("RANK", "0")) != 0:
         return
     from bevy_b200 import scenes
@@ -543,6 +548,44 @@ def measure_pcie(torch, dev, stream):
     return out
 
 
+DUMP_ROWS = 1 << 18             # per-row columns: a seeded sample of this many rows (every row when there are fewer)
+DUMP_LIST_ENTRIES = 1 << 21     # visible lists, and again cluster index lists: at most this many entries over all views
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, ctx, n, V):
+    """Writes what the last step computed, as a caller of the device-resident path downloads it: GlobalTransforms, both
+    change columns, ViewVisibility, the sorted visible lists, the cluster lists and the frame stats.  Long outputs are
+    reduced to a fixed seeded sample (the sampled row ids go to rows.npy), so that the files stay below DUMP_MAX_BYTES at
+    any scene size and two builds run with the same arguments can be compared file for file."""
+    def sample(count, cap, seed):
+        if count <= cap:
+            return np.arange(count)
+        return np.sort(np.random.default_rng(seed).choice(count, cap, replace=False))
+
+    rows = sample(n, DUMP_ROWS, 0)
+    gt, gt_changed = ctx.download_global_transforms(0, n)
+    vv, vv_changed = ctx.download_view_visibility(0, n)
+    stats = ctx.download_frame_stats()
+    out = {"rows": rows.astype(np.float64), "global_transform": gt[rows],
+           "global_transform_changed": gt_changed[rows].astype(np.float32),
+           "view_visibility": vv[rows].astype(np.float32), "view_visibility_changed": vv_changed[rows].astype(np.float32),
+           "visible_count": np.array(stats.visible_count[:V], np.float64),
+           "cluster_index_count": np.array(stats.cluster_index_count[:V], np.float64),
+           "cluster_farthest_z": np.array(stats.cluster_farthest_z[:V], np.float32),
+           "changed_count": np.array([stats.gt_changed_count, stats.vv_changed_count], np.float64)}
+    for v in range(V):
+        vis = ctx.download_visible(v)
+        out[f"visible_rows_view{v}"] = vis[sample(len(vis), DUMP_LIST_ENTRIES // V, 1 + v)].astype(np.float64)
+        offsets, idx = ctx.download_clusters(v)
+        out[f"cluster_offsets_view{v}"] = offsets[:ctx.cluster_dims(v) + 1].astype(np.float64)
+        out[f"cluster_indices_view{v}"] = idx[sample(len(idx), DUMP_LIST_ENTRIES // V, 1 + V + v)].astype(np.float64)
+    assert sum(a.nbytes for a in out.values()) <= DUMP_MAX_BYTES
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def measure_next_rows(torch, bb, rig, tile_ms, expand_ms, cluster_ms, e2e_resident_ms, W):
     """Cost of the SURVEY.md 8(f) rows on the bench workload (1 GPU): stage times with the row switched on against the
     base numbers measured above (same CUDA-event stage timers), plus the e2e frame when the shim takes the added /
@@ -763,6 +806,8 @@ def main():
     value_launches = (abi.kernel_launch_count() - launches0) / K
     ts1 = time.time()
     clocks = sampler.stop(ts0, ts1)
+    if args.dump_outputs and rank == 0:          # N > 1: rank 0's rows, and the cluster lists every rank holds
+        dump_outputs(args.dump_outputs, ctx, n, V)
     if not args.no_parity:
         fchk = W + K
         if fchk % WIN == 0:        # slot 0's recorded constants carry the feedback of the frame before the recording run

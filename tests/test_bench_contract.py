@@ -4,6 +4,9 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -34,6 +37,41 @@ def test_reference_arm_prints_one_contract_line():
     res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2"], env=env,
                          capture_output=True, text=True, timeout=120, cwd=ROOT)
     assert res.returncode == 0 and res.stdout.strip() == ""
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_same_on_every_run(tmp_path):
+    """--dump-outputs: the last timed step's results as float32 / float64 .npy files, under 64 MB, bit for bit the same on
+    two runs with the same arguments; --steps sets the number of timed steps."""
+    n = 300 * 255 + 32
+    dumps = []
+    for run in range(2):
+        out = tmp_path / f"run{run}"
+        res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "7", "--warmup", "3", "--trees", "300",
+                              "--lights", "32", "--no-cpu-baseline", "--no-next-rows", "--dump-outputs", str(out)],
+                             capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert res.returncode == 0, res.stderr[-3000:]
+        d = json.loads(res.stdout.strip().splitlines()[-1])
+        assert d["steps"] == 7 and d["parity_checked"] is True
+        files = {p.stem: np.load(p) for p in sorted(out.glob("*.npy"))}
+        assert all(a.dtype in (np.float32, np.float64) for a in files.values())
+        assert sum(a.nbytes for a in files.values()) <= 64 << 20
+        dumps.append(files)
+    a, b = dumps
+    assert a.keys() == b.keys()
+    for k in a:
+        assert a[k].shape == b[k].shape and a[k].tobytes() == b[k].tobytes(), k
+    assert np.array_equal(a["rows"], np.arange(n)) and a["global_transform"].shape == (n, 12)
+    assert a["view_visibility"].any() and a["visible_count"].sum() > 0
+    for v in range(4):
+        assert len(a[f"visible_rows_view{v}"]) == a["visible_count"][v]
+        assert a[f"cluster_offsets_view{v}"][-1] == a["cluster_index_count"][v] == len(a[f"cluster_indices_view{v}"])
+
+
+def test_reference_arm_refuses_dump_outputs(tmp_path):
+    res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=120, cwd=ROOT)
+    assert res.returncode != 0 and "--dump-outputs" in res.stderr and not any(tmp_path.iterdir())
 
 
 def test_b200_arm_fails_loudly_without_a_gpu():
