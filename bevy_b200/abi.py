@@ -16,6 +16,9 @@ STAGE_CLUSTER = STAGE_CLUSTER_ASSIGN | STAGE_CLUSTER_LISTS
 STAGE_ALL = 0xF
 MAX_VIEWS = 8
 MAX_CLUSTERS = 4096
+# ClusterableObjectType::ordering().0 of the objects b200vis_set_clusterable_objects takes (assign.rs:115-131)
+CLUSTERABLE_RECT_LIGHT, CLUSTERABLE_REFLECTION_PROBE, CLUSTERABLE_IRRADIANCE_VOLUME, CLUSTERABLE_DECAL = 2, 3, 4, 5
+BINDINGS_OFF, BINDINGS_STORAGE, BINDINGS_UNIFORM = 0, 1, 2
 
 ERR_NAMES = {1: "INVALID_ARG", 2: "CUDA", 3: "OUT_OF_MEMORY", 4: "HIERARCHY_CYCLE", 5: "PARENT_OUT_OF_RANGE",
              6: "CAPACITY", 7: "NOT_READY", 8: "UNSUPPORTED"}
@@ -139,6 +142,7 @@ _SIGNATURES = {
     "b200vis_update_camera": (C.c_int32, [_vp, C.c_uint32, _P(CameraDesc), _P(ClusterConfig), _P(ClusterFeedback), _P(ClusterView)]),
     "b200vis_download_frame": (C.c_int32, [_vp, _P(FrameStats), _vp, C.c_uint32, _vp, _vp, C.c_uint32]),
     "b200vis_set_lights": (C.c_int32, [_vp, C.c_uint32, _vp, _vp, _vp]),
+    "b200vis_set_clusterable_objects": (C.c_int32, [_vp, C.c_uint32, _vp, _vp, _vp, _vp]),
     "b200vis_set_cluster_view": (C.c_int32, [_vp, C.c_uint32, _P(ClusterView)]),
     "b200vis_record_frame_constants": (C.c_int32, [_vp, _P(C.c_uint32)]),
     "b200vis_use_recorded_frame_constants": (C.c_int32, [_vp, C.c_int32]),
@@ -441,6 +445,17 @@ class Context:
     def set_lights(self, light_row, light_range, layer_mask=None):
         r = _arr(light_row, np.uint32); g = _arr(light_range, np.float32); l = _arr(layer_mask, np.uint64)
         self._check(self._lib.b200vis_set_lights(self._h, len(r), _ptr(r), _ptr(g), _ptr(l)))
+
+    def set_clusterable_objects(self, kind, row, rect_range=None, layer_mask=None):
+        """Rect lights, light probes and clustered decals (kinds CLUSTERABLE_*), grouped in the reference's push order; object j
+        becomes cluster ordinal n_lights + j.  rect_range / layer_mask: one entry per object, read for rect lights only.
+        Empty arrays remove the objects."""
+        k = _arr(kind, np.uint32); r = _arr(row, np.uint32)
+        assert len(k) == len(r)
+        g = _arr(rect_range, np.float32); l = _arr(layer_mask, np.uint64)
+        assert g is None or len(g) == len(k)
+        assert l is None or len(l) == len(k)
+        self._check(self._lib.b200vis_set_clusterable_objects(self._h, len(k), _ptr(k), _ptr(r), _ptr(g), _ptr(l)))
 
     def cluster_dims(self, view):
         """Number of clusters of the view's current grid (0 = clustering off)."""

@@ -137,9 +137,15 @@ struct b200vis_ctx {
 
     // lights + clusters
     std::vector<uint32_t> h_light_row; std::vector<float> h_light_range;   // host copies (b200vis_set_shadow_lights resolves ordinals)
+    std::vector<uint64_t> h_light_layers;                                  // empty = default layer (the light blocks are rebuilt from these)
     Lights lights{}; uint32_t *d_light_row = nullptr; float *d_light_range = nullptr; uint64_t *d_light_layers = nullptr;
     ClusterBufs cl{}; uint32_t *d_slab = nullptr; void *ext_send = nullptr, *ext_recv = nullptr;
     size_t slab_bytes = 0;
+    // clusterable objects (b200vis_set_clusterable_objects): cluster ordinals [lights.n, lights.n + h_obj_kind.size())
+    std::vector<uint8_t> h_obj_kind; std::vector<float> h_obj_range; std::vector<uint64_t> h_obj_layers;
+    uint32_t *d_obj_row = nullptr;      // [max_lights] object j's row
+    uint8_t *d_ord_kind = nullptr;      // [cl.max_lights] kind of every ordinal (0 = point light), rewritten when an ordinal moves
+    uint32_t n_objects() const { return (uint32_t)h_obj_kind.size(); }
 
     // result sink (mapped pinned host memory written by publish kernels)
     b200vis_result_sink sink{}; bool have_sink = false;
@@ -212,7 +218,7 @@ extern "C" void b200vis_destroy(b200vis_ctx *ctx) {
                    ctx->bind.oc, ctx->bind.il, ctx->bind.count, ctx->d_bind_map,
                    ctx->d_range_se, ctx->d_range_ua, ctx->d_range_views, ctx->d_visibility, ctx->d_iv_changed,
                    ctx->d_shadow_lights, ctx->d_caster, ctx->shadow.mask, ctx->shadow.chunk_count, ctx->shadow.lists,
-                   ctx->shadow.count, ctx->shadow.active};
+                   ctx->shadow.count, ctx->shadow.active, ctx->d_obj_row, ctx->d_ord_kind};
     for (void *p : dev) if (p) cudaFree(p);
     for (int i = 0; i < b200vis_ctx::kRing; ++i) {
         if (ctx->h_ring[i]) cudaFreeHost(ctx->h_ring[i]);
@@ -969,10 +975,33 @@ extern "C" int32_t b200vis_update_camera(b200vis_ctx *ctx, uint32_t view, const 
     return B200VIS_OK;
 }
 
+// The light blocks of the three frame slots: stale snapshots out, the ranges and layer masks of every ordinal in (point lights,
+// then the clusterable objects), and the kind byte of every ordinal when objects are set.  Rare (set time only): the tail of
+// the frame in flight is joined first.
+static int32_t write_light_blocks(b200vis_ctx *ctx) {
+    const int32_t jrc = join_all(ctx); if (jrc) return jrc;
+    const uint32_t cap = ctx->cl.max_lights, nl = ctx->lights.n, no = ctx->n_objects();
+    std::vector<uint8_t> blk(ctx->lrec_bytes, 0);
+    float *rg = reinterpret_cast<float *>(blk.data() + (size_t)cap * 16);
+    uint64_t *ly = reinterpret_cast<uint64_t *>(blk.data() + (size_t)cap * 20);
+    for (uint32_t i = 0; i < nl; ++i) { rg[i] = ctx->h_light_range[i]; ly[i] = ctx->h_light_layers.empty() ? 1ull : ctx->h_light_layers[i]; }
+    for (uint32_t j = 0; j < no; ++j) { rg[nl + j] = ctx->h_obj_range[j]; ly[nl + j] = ctx->h_obj_layers[j]; }
+    CU(cudaStreamSynchronize(ctx->stream));
+    for (int k = 0; k < 3; ++k) CU(cudaMemcpy(ctx->d_lrec + k * ctx->lrec_bytes, blk.data(), ctx->lrec_bytes, cudaMemcpyHostToDevice));
+    if (no) {
+        std::vector<uint8_t> kinds(nl, (uint8_t)kKindPoint);
+        kinds.insert(kinds.end(), ctx->h_obj_kind.begin(), ctx->h_obj_kind.end());
+        CU(cudaMemcpy(ctx->d_ord_kind, kinds.data(), kinds.size(), cudaMemcpyHostToDevice));
+    }
+    return B200VIS_OK;
+}
+
 extern "C" int32_t b200vis_set_lights(b200vis_ctx *ctx, uint32_t n_lights, const uint32_t *light_row, const float *range,
                                       const uint64_t *layer_mask) {
     CHECK_CTX();
     if (n_lights > ctx->cfg.max_lights) return fail(ctx, B200VIS_ERR_CAPACITY, "set_lights: %u > max_lights %u", n_lights, ctx->cfg.max_lights);
+    if (n_lights + ctx->n_objects() > ctx->cfg.max_lights)
+        return fail(ctx, B200VIS_ERR_CAPACITY, "set_lights: %u lights + %u clusterable objects > max_lights %u", n_lights, ctx->n_objects(), ctx->cfg.max_lights);
     if (n_lights && (!light_row || !range)) return fail(ctx, B200VIS_ERR_INVALID_ARG, "set_lights: null");
     for (uint32_t i = 0; i < n_lights; ++i)
         if (light_row[i] >= ctx->cfg.max_entities) return fail(ctx, B200VIS_ERR_INVALID_ARG, "set_lights: light %u row %u out of range", i, light_row[i]);
@@ -980,20 +1009,49 @@ extern "C" int32_t b200vis_set_lights(b200vis_ctx *ctx, uint32_t n_lights, const
     CU(cudaMemcpyAsync(ctx->d_light_range, range, (size_t)n_lights * 4, cudaMemcpyHostToDevice, ctx->stream));
     if (layer_mask) CU(cudaMemcpyAsync(ctx->d_light_layers, layer_mask, (size_t)n_lights * 8, cudaMemcpyHostToDevice, ctx->stream));
     ctx->h_light_row.assign(light_row, light_row + n_lights); ctx->h_light_range.assign(range, range + n_lights);
+    if (layer_mask) ctx->h_light_layers.assign(layer_mask, layer_mask + n_lights); else ctx->h_light_layers.clear();
     ctx->lights.n = n_lights; ctx->lights.row = ctx->d_light_row; ctx->lights.range = ctx->d_light_range;
     ctx->lights.layers = layer_mask ? ctx->d_light_layers : nullptr;
     ctx->lights_tag_dirty = true;
-    {   // the light blocks: stale snapshots out, ranges and layer masks in (rare: the tail of the frame in flight is joined first)
-        const int32_t jrc = join_all(ctx); if (jrc) return jrc;
-        const uint32_t cap = ctx->cl.max_lights;
-        std::vector<uint8_t> blk(ctx->lrec_bytes, 0);
-        float *rg = reinterpret_cast<float *>(blk.data() + (size_t)cap * 16);
-        uint64_t *ly = reinterpret_cast<uint64_t *>(blk.data() + (size_t)cap * 20);
-        for (uint32_t i = 0; i < n_lights; ++i) { rg[i] = range[i]; ly[i] = layer_mask ? layer_mask[i] : 1ull; }
-        CU(cudaStreamSynchronize(ctx->stream));
-        for (int k = 0; k < 3; ++k) CU(cudaMemcpy(ctx->d_lrec + k * ctx->lrec_bytes, blk.data(), ctx->lrec_bytes, cudaMemcpyHostToDevice));
+    return write_light_blocks(ctx);   // the objects' ordinals follow the new point-light count
+}
+
+extern "C" int32_t b200vis_set_clusterable_objects(b200vis_ctx *ctx, uint32_t n, const uint32_t *kind, const uint32_t *row,
+                                                   const float *range, const uint64_t *layer_mask) {
+    CHECK_CTX();
+    if (n && ctx->cfg.world_size > 1)
+        return fail(ctx, B200VIS_ERR_UNSUPPORTED, "set_clusterable_objects: world_size %u > 1 (rank-major ordinals would break the grouping by kind)", ctx->cfg.world_size);
+    if (ctx->lights.n + n > ctx->cfg.max_lights)
+        return fail(ctx, B200VIS_ERR_CAPACITY, "set_clusterable_objects: %u lights + %u objects > max_lights %u", ctx->lights.n, n, ctx->cfg.max_lights);
+    if (n && (!kind || !row)) return fail(ctx, B200VIS_ERR_INVALID_ARG, "set_clusterable_objects: null");
+    if (n && ctx->bind.mode == B200VIS_BINDINGS_UNIFORM)
+        return fail(ctx, B200VIS_ERR_INVALID_ARG, "set_clusterable_objects: uniform cluster bindings hold point and spot lights only");
+    uint32_t last_group = 0;
+    for (uint32_t j = 0; j < n; ++j) {
+        const uint32_t k = kind[j];
+        if (k == 1u) return fail(ctx, B200VIS_ERR_UNSUPPORTED, "set_clusterable_objects: object %u is a spot light", j);
+        if (k < B200VIS_CLUSTERABLE_RECT_LIGHT || k > B200VIS_CLUSTERABLE_DECAL)
+            return fail(ctx, B200VIS_ERR_INVALID_ARG, "set_clusterable_objects: object %u has kind %u", j, k);
+        // push order (assign.rs:231-295): rect lights, then probes and volumes (one query, interleaved), then decals
+        const uint32_t group = k == B200VIS_CLUSTERABLE_RECT_LIGHT ? 0u : k == B200VIS_CLUSTERABLE_DECAL ? 2u : 1u;
+        if (group < last_group) return fail(ctx, B200VIS_ERR_INVALID_ARG, "set_clusterable_objects: object %u (kind %u) is out of push order", j, k);
+        last_group = group;
+        if (row[j] >= ctx->cfg.max_entities) return fail(ctx, B200VIS_ERR_INVALID_ARG, "set_clusterable_objects: object %u row %u out of range", j, row[j]);
+        if (k == B200VIS_CLUSTERABLE_RECT_LIGHT && !range) return fail(ctx, B200VIS_ERR_INVALID_ARG, "set_clusterable_objects: rect lights need a range");
     }
-    return B200VIS_OK;
+    if (n && !ctx->d_obj_row) {
+        CU(dalloc(&ctx->d_obj_row, std::max<uint32_t>(ctx->cfg.max_lights, 1)));
+        CU(dalloc(&ctx->d_ord_kind, ctx->cl.max_lights));
+    }
+    const int32_t jrc = join_all(ctx); if (jrc) return jrc;   // the frame in flight may still read the rows
+    CU(cudaStreamSynchronize(ctx->stream));
+    if (n) CU(cudaMemcpy(ctx->d_obj_row, row, (size_t)n * 4, cudaMemcpyHostToDevice));
+    ctx->h_obj_kind.resize(n); ctx->h_obj_range.assign(n, 0.0f); ctx->h_obj_layers.assign(n, 1ull);
+    for (uint32_t j = 0; j < n; ++j) {
+        ctx->h_obj_kind[j] = (uint8_t)kind[j];
+        if (kind[j] == B200VIS_CLUSTERABLE_RECT_LIGHT) { ctx->h_obj_range[j] = range[j]; if (layer_mask) ctx->h_obj_layers[j] = layer_mask[j]; }
+    }
+    return write_light_blocks(ctx);
 }
 
 extern "C" int32_t b200vis_cluster_view_dims(const b200vis_ctx *ctx, uint32_t view, uint32_t dims[3]) {
@@ -1385,15 +1443,34 @@ extern "C" int32_t b200vis_run(b200vis_ctx *ctx, uint32_t stages) {
     }
     Lights lights = ctx->lights;
     lights.snap = nullptr;
+    // Clusterable objects: snapshotted into the frame slot beside the point lights, and then every ordinal's sphere (the
+    // objects' ranges included) is read through that slot.  Without objects nothing here is launched.
+    ClusterObjects objs{};
+    objs.n = has_assign ? ctx->n_objects() : 0u; objs.base = ctx->lights.n; objs.row = ctx->d_obj_row;
+    objs.kind = objs.n ? ctx->d_ord_kind + ctx->lights.n : nullptr;
+    float *slot_range = reinterpret_cast<float *>(ctx->d_lrec + (size_t)cslot * ctx->lrec_bytes + (size_t)ctx->cl.max_lights * 16);
     cudaStream_t tail = st;
     if (pipelined) {
         lights.snap = ctx->light_snap_slot(cslot);
         if (!tile_snap) launch_snapshot_lights(st, R, lights, const_cast<float4 *>(lights.snap));
+        launch_snapshot_objects(st, R, objs, const_cast<float4 *>(lights.snap), slot_range);
         if (pe) CU(cudaEventRecord(pe[1], st));
         CU(cudaEventRecord(ctx->ev_tile, st));
         tail = ctx->side_stream;
         CU(cudaStreamWaitEvent(tail, ctx->ev_tile, 0));
-    } else if (pe) CU(cudaEventRecord(pe[1], st));
+    } else {
+        if (objs.n) {      // serial: the same snapshot, behind whatever this call ran on the stream
+            lights.snap = ctx->light_snap_slot(cslot);
+            launch_snapshot_lights(st, R, lights, const_cast<float4 *>(lights.snap));
+            launch_snapshot_objects(st, R, objs, const_cast<float4 *>(lights.snap), slot_range);
+        }
+        if (pe) CU(cudaEventRecord(pe[1], st));
+    }
+    if (objs.n) {
+        lights.n += objs.n;
+        lights.range = slot_range;
+        lights.layers = reinterpret_cast<const uint64_t *>(ctx->d_lrec + (size_t)cslot * ctx->lrec_bytes + (size_t)ctx->cl.max_lights * 20);
+    }
     if (pe) CU(cudaEventRecord(pe[2], tail));
     // Multi-GPU: the cluster exchange is the one step of the tail that waits on other GPUs, so it goes FIRST -- assign and
     // the slab push / all-gather are issued before the visible-list expansion (they do not depend on it), and the peers'
@@ -1494,8 +1571,11 @@ extern "C" int32_t b200vis_run(b200vis_ctx *ctx, uint32_t stages) {
     }
     if ((stages & B200VIS_STAGE_CLUSTER_LISTS) && !fused_clusters)
         launch_cluster_lists(ctail, fc, cl, ctx->d_stats, ctx->cfg.max_views);
-    if ((stages & B200VIS_STAGE_CLUSTER_LISTS) && ctx->bind.mode)
-        launch_pack_cluster_bindings(ctail, fc, cl, ctx->bind, ctx->cfg.max_views);
+    if ((stages & B200VIS_STAGE_CLUSTER_LISTS) && ctx->bind.mode) {
+        BindingBufs bb = ctx->bind;
+        bb.kind = ctx->n_objects() ? ctx->d_ord_kind : nullptr;
+        launch_pack_cluster_bindings(ctail, fc, cl, bb, ctx->cfg.max_views);
+    }
     if (branch) { CU(cudaEventRecord(ctx->ev_clus, ctail)); CU(cudaStreamWaitEvent(tail, ctx->ev_clus, 0)); }   // the branches meet
     // (b200vis_step with clusters runs CLUSTER right behind PROPAGATE|CULL: that run publishes the stats block once for both)
     if (ctx->have_sink && (do_cull || (stages & B200VIS_STAGE_CLUSTER_LISTS)) && !(ctx->step_defers_stats && !(stages & B200VIS_STAGE_CLUSTER_LISTS)))
@@ -1801,6 +1881,8 @@ extern "C" int32_t b200vis_set_cluster_bindings(b200vis_ctx *ctx, uint32_t mode,
     CHECK_CTX_JOIN();
     if (mode > B200VIS_BINDINGS_UNIFORM) return fail(ctx, B200VIS_ERR_INVALID_ARG, "set_cluster_bindings: mode %u", mode);
     if (gpu_index_of_light && !n_map) return fail(ctx, B200VIS_ERR_INVALID_ARG, "set_cluster_bindings: empty index map");
+    if (mode == B200VIS_BINDINGS_UNIFORM && ctx->n_objects())
+        return fail(ctx, B200VIS_ERR_INVALID_ARG, "set_cluster_bindings: uniform bindings with %u clusterable objects set", ctx->n_objects());
     const size_t V = ctx->cfg.max_views;
     if (mode && !ctx->bind.oc) {
         ctx->bind.il_stride = std::max<uint32_t>(ctx->cl.index_cap, 4096u);
@@ -2042,7 +2124,7 @@ extern "C" int32_t b200vis_step(b200vis_ctx *ctx, uint32_t n_changed, const uint
     if (n_changed && (rc = b200vis_upload_transforms_scattered(ctx, n_changed, rows, trs))) return rc;
     lap(0);
     if ((rc = b200vis_set_view_count(ctx, n_cameras))) return rc;
-    const bool clusters = cfg != nullptr && ctx->lights.n > 0;
+    const bool clusters = cfg != nullptr && ctx->lights.n + ctx->n_objects() > 0;
     // frusta first, so the tile pass starts at once; the per-view cluster prologue (plane tables, z thresholds: tens of
     // microseconds of host maths) is computed while that kernel runs, then the cluster stage is enqueued behind it
     for (uint32_t v = 0; v < n_cameras; ++v)

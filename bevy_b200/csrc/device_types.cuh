@@ -185,6 +185,16 @@ __device__ __forceinline__ unsigned long long light_layers_of(const Lights &L, u
 }
 #endif
 
+// b200vis_set_clusterable_objects: object j (row[j], kind[j]) is cluster ordinal base + j, base = the point-light count.
+// k_snapshot_objects writes its (translation, visible) and -- for probes and decals -- its radius into the frame slot's
+// light block, so that the cluster kernels read every ordinal's sphere the same way.
+constexpr uint32_t kKindPoint = 0, kKindRect = 2, kKindReflectionProbe = 3, kKindIrradianceVolume = 4, kKindDecal = 5;
+struct ClusterObjects {
+    uint32_t n, base;
+    const uint32_t *row;
+    const uint8_t *kind;     // [n]
+};
+
 struct ClusterBufs {
     uint32_t words;          // mask words per rank = ceil(max_lights/32)
     uint32_t max_lights;     // per rank
@@ -237,6 +247,7 @@ struct BindingBufs {
     uint32_t *il;            // [V][il_stride]         storage: one u32 per index; uniform: the first 4096 words
     uint32_t il_stride;
     uint32_t *count;         // [V][2] n_offsets, n_indices
+    const uint8_t *kind;     // per cluster ordinal: kKind* (storage mode splits the counts by kind), or nullptr (all point lights)
 };
 
 }  // namespace b200vis

@@ -3234,6 +3234,37 @@ __global__ void k_snapshot_lights(Rows R, Lights L, float4 *__restrict__ snap) {
     snap[li] = make_float4(R.gt0[row].w, R.gt1[row].w, R.gt2[row].w, (R.state[row] & 1u) ? 1.0f : 0.0f);
 }
 
+// GlobalTransform::radius_vec3a(h) = (matrix3 * h).length() (global_transform.rs:252-254) on the row form of the matrix:
+// Mat3A * Vec3A = ((X*h.x) + (Y*h.y)) + (Z*h.z) lane-wise, Vec3A::length = sqrt((x*x + y*y) + z*z) -- the expression the
+// cull phase evaluates for an Aabb's half extents (glam order unverified, DESIGN.md §5)
+__device__ __forceinline__ float radius_vec3a(float4 r0, float4 r1, float4 r2, float hx, float hy, float hz) {
+    const float vx = (r0.x * hx + r0.y * hy) + r0.z * hz;
+    const float vy = (r1.x * hx + r1.y * hy) + r1.z * hz;
+    const float vz = (r2.x * hx + r2.y * hy) + r2.z * hz;
+    return sqrtf((vx * vx + vy * vy) + vz * vz);
+}
+
+// The clusterable objects of b200vis_set_clusterable_objects at the light snapshot's stream position: (translation, visible)
+// of ordinal base + j into `snap`, and the radius of the kinds that derive it from GlobalTransform into `range`
+// (assign.rs:256-295).  Rect-light ranges were written into every frame slot at set time.
+__global__ void k_snapshot_objects(Rows R, ClusterObjects O, float4 *__restrict__ snap, float *__restrict__ range) {
+    const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= O.n) return;
+    const uint32_t row = O.row[j], kind = O.kind[j];
+    const float4 r0 = R.gt0[row], r1 = R.gt1[row], r2 = R.gt2[row];
+    snap[O.base + j] = make_float4(r0.w, r1.w, r2.w, (R.state[row] & 1u) ? 1.0f : 0.0f);
+    if (kind == kKindReflectionProbe || kind == kKindIrradianceVolume) {
+        range[O.base + j] = radius_vec3a(r0, r1, r2, 1.0f, 1.0f, 1.0f);           // transform.radius_vec3a(Vec3A::ONE)
+    } else if (kind == kKindDecal) {
+        // transform.scale().length() (global_transform.rs:240-248): the axis lengths, the first one times copysign(1, det),
+        // whose sign squares away exactly -- so the determinant is not needed
+        const float lx = sqrtf((r0.x * r0.x + r1.x * r1.x) + r2.x * r2.x);
+        const float ly = sqrtf((r0.y * r0.y + r1.y * r1.y) + r2.y * r2.y);
+        const float lz = sqrtf((r0.z * r0.z + r1.z * r1.z) + r2.z * r2.z);
+        range[O.base + j] = sqrtf((lx * lx + ly * ly) + lz * lz);
+    }
+}
+
 // ---- result sink: coalesced copies of a frame's results into mapped pinned host memory ----------------------
 // visible lists: grid (blocks, views), grid-stride over the view's count
 __global__ void k_publish_visible(const uint32_t *__restrict__ lists, uint32_t list_stride, const DevStats *__restrict__ stats,
@@ -3623,8 +3654,19 @@ __global__ void k_pack_cluster_bindings(const FrameConsts *__restrict__ fc, Clus
     };
     if (bb.mode == 1u) {   // storage: (offset, point, spot, rect | probes, volumes, decals, 0) per cluster (:636-652)
         for (uint32_t c = tid; c < nc; c += nth) {
-            reinterpret_cast<uint4 *>(oc)[c * 2] = make_uint4(off[c], off[c + 1] - off[c], 0u, 0u);
-            reinterpret_cast<uint4 *>(oc)[c * 2 + 1] = make_uint4(0u, 0u, 0u, 0u);
+            const uint32_t len = off[c + 1] - off[c];
+            if (bb.kind == nullptr) {
+                reinterpret_cast<uint4 *>(oc)[c * 2] = make_uint4(off[c], len, 0u, 0u);
+                reinterpret_cast<uint4 *>(oc)[c * 2 + 1] = make_uint4(0u, 0u, 0u, 0u);
+                continue;
+            }
+            // ObjectsInClusterCpu::add_* (bevy_light/src/cluster/mod.rs:478-512): one counter per kind; the entries that did
+            // not fit max_cluster_indices count as point lights
+            uint32_t n_kind[6] = {0u, 0u, 0u, 0u, 0u, 0u};
+            for (uint32_t i = off[c]; i < min(off[c + 1], avail); ++i) ++n_kind[min((uint32_t)bb.kind[idx[i]], 5u)];
+            const uint32_t objects = n_kind[kKindRect] + n_kind[kKindReflectionProbe] + n_kind[kKindIrradianceVolume] + n_kind[kKindDecal];
+            reinterpret_cast<uint4 *>(oc)[c * 2] = make_uint4(off[c], len - objects, 0u, n_kind[kKindRect]);
+            reinterpret_cast<uint4 *>(oc)[c * 2 + 1] = make_uint4(n_kind[kKindReflectionProbe], n_kind[kKindIrradianceVolume], n_kind[kKindDecal], 0u);
         }
         for (uint32_t i = tid; i < avail; i += nth) il[i] = gpu_index(idx[i]);
         if (tid == 0) { bb.count[v * 2] = nc; bb.count[v * 2 + 1] = avail; }
@@ -4121,6 +4163,9 @@ void launch_tag_lights(cudaStream_t st, const Rows &R, const Lights &L, uint32_t
 }
 void launch_snapshot_lights(cudaStream_t st, const Rows &R, const Lights &L, float4 *snap) {
     if (L.n) { ++g_launches; k_snapshot_lights<<<cdiv(L.n, 128), 128, 0, st>>>(R, L, snap); }
+}
+void launch_snapshot_objects(cudaStream_t st, const Rows &R, const ClusterObjects &O, float4 *snap, float *range) {
+    if (O.n) { ++g_launches; k_snapshot_objects<<<cdiv(O.n, 128), 128, 0, st>>>(R, O, snap, range); }
 }
 void launch_writeback_columns(cudaStream_t st, const Rows &R, float *host_gt, uint32_t stride, uint32_t *host_gt_bits, uint8_t *host_vv,
                               uint32_t *host_vv_bits, uint8_t *vv_shadow) {

@@ -35,6 +35,7 @@ void launch_publish_clusters(cudaStream_t st, const FrameConsts *fc, const Clust
                              uint32_t host_cap, const DevStats *stats, uint32_t *host_stats, uint32_t changed_slot, uint32_t frame, uint32_t max_views);
 void launch_tag_lights(cudaStream_t st, const Rows &R, const Lights &L, uint32_t *light_ord, uint32_t *all_tagged);
 void launch_snapshot_lights(cudaStream_t st, const Rows &R, const Lights &L, float4 *snap);
+void launch_snapshot_objects(cudaStream_t st, const Rows &R, const ClusterObjects &O, float4 *snap, float *range);
 void launch_writeback_columns(cudaStream_t st, const Rows &R, float *host_gt, uint32_t stride, uint32_t *host_gt_bits, uint8_t *host_vv,
                               uint32_t *host_vv_bits, uint8_t *vv_shadow);
 void launch_record_push(cudaStream_t st, const uint32_t *block, uint32_t block_words, const ClusterBufs &cb);

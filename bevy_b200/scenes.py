@@ -252,6 +252,53 @@ def propagate_bench_scene():
                  cameras=[_camera(0.0)], roots=np.array(roots, np.uint32))
 
 
+RECT_LIGHT, REFLECTION_PROBE, IRRADIANCE_VOLUME, DECAL = 2, 3, 4, 5   # ClusterableObjectType::ordering().0
+
+
+def add_clusterable_objects(scene, n_rect=64, n_probe=128, n_decal=256, seed=7, hidden_frac=0.1,
+                            rect_layer_choices=(1, 2, 3)):
+    """Appends rect lights, light probes (reflection probes and irradiance volumes interleaved) and clustered decals to
+    `scene`, in the reference's push order (assign.rs:231-295), and records them as scene.obj_kind / obj_row / obj_range /
+    obj_layers.  Each object is a child of a random hierarchy root, so its GlobalTransform changes whenever the roots move,
+    with a random rotation and a non-uniform scale whose x is negated for every third object (negative determinant).  All
+    carry the unit-cube Aabb of add_light_probe_and_decal_aabbs (bevy_light/src/cluster/mod.rs:520-537), so the cull decides
+    their ViewVisibility; `hidden_frac` of them are not InheritedVisibility-visible.  Rect lights get a log-uniform range and
+    a RenderLayers mask drawn from `rect_layer_choices` (also their row's layer mask); probes and decals the default layer.
+    The scene's columns are replaced by longer ones; the scene is returned."""
+    rng = np.random.default_rng(seed)
+    n_obj = n_rect + n_probe + n_decal
+    kind = np.concatenate([np.full(n_rect, RECT_LIGHT), rng.choice([REFLECTION_PROBE, IRRADIANCE_VOLUME], n_probe),
+                           np.full(n_decal, DECAL)]).astype(np.uint32)
+    n0 = scene.n
+    roots = scene.roots if scene.roots is not None and len(scene.roots) else np.zeros(0, np.uint32)
+    parent = roots[rng.integers(0, len(roots), n_obj)].astype(np.uint32) if len(roots) else np.full(n_obj, NO_PARENT, np.uint32)
+    s = rng.uniform(0.5, 3.0, (n_obj, 3))
+    s[::3, 0] *= -1.0
+    trs = _trs(rng.uniform(-3.0, 3.0, (n_obj, 3)).astype(np.float32), random_unit_quats(rng, n_obj).astype(np.float32),
+               s.astype(np.float32))
+    bounds = np.zeros((n_obj, 6), np.float32); bounds[:, 3:6] = 0.5
+    flags = np.full(n_obj, F_INHERITED_VISIBLE | F_HAS_AABB, np.uint8)
+    flags[rng.random(n_obj) < hidden_frac] = F_HAS_AABB
+    obj_range = np.zeros(n_obj, np.float32)
+    obj_range[:n_rect] = np.exp(rng.uniform(math.log(0.5), math.log(15.0), n_rect))
+    obj_layers = np.ones(n_obj, np.uint64)
+    obj_layers[:n_rect] = np.asarray(rect_layer_choices, np.uint64)[rng.integers(0, len(rect_layer_choices), n_rect)]
+    layer_mask = np.ones(n0, np.uint64) if scene.layer_mask is None else scene.layer_mask
+    scene.parent = np.concatenate([scene.parent, parent])
+    scene.trs = np.concatenate([scene.trs, trs])
+    scene.bounds = np.concatenate([scene.bounds, bounds])
+    scene.flags = np.concatenate([scene.flags, flags])
+    scene.class_mask = np.concatenate([scene.class_mask, np.full(n_obj, CLASS_LIGHT, np.uint8)])
+    scene.entity_bits = np.concatenate([scene.entity_bits, _entity_bits(n_obj, int(scene.entity_bits.max()) + 1 if n0 else 0)])
+    scene.layer_mask = np.concatenate([layer_mask, obj_layers])
+    if scene.range_mask is not None:
+        scene.range_mask = np.concatenate([scene.range_mask, np.zeros(n_obj, np.uint32)])
+    scene.obj_kind, scene.obj_row = kind, (n0 + np.arange(n_obj)).astype(np.uint32)
+    scene.obj_range, scene.obj_layers = obj_range, obj_layers
+    scene.name = f"{scene.name}_O{n_rect}r{n_probe}p{n_decal}d"
+    return scene
+
+
 # ---- per-frame animation ---------------------------------------------------------------------
 def advance_cameras(scene, delta=0.15 / 60.0):
     """move_camera (many_cubes.rs:590-603): rotate_z(delta) then rotate_x(delta); Transform::rotate

@@ -84,7 +84,8 @@ typedef struct b200vis_ctx b200vis_ctx;
 typedef struct b200vis_config {
     int32_t  device;              /* CUDA device ordinal */
     uint32_t max_entities;        /* row capacity */
-    uint32_t max_lights;          /* point lights this context (this rank's shard) may hold */
+    uint32_t max_lights;          /* cluster ordinals this context (this rank's shard) may hold: point lights plus the
+                                     objects of b200vis_set_clusterable_objects */
     uint32_t max_views;           /* <= B200VIS_MAX_VIEWS */
     uint32_t max_cluster_indices; /* per-view capacity of the cluster index list (0 => 1<<20) */
     uint32_t world_size;          /* ranks sharing the cluster exchange (0/1 => single GPU) */
@@ -247,6 +248,28 @@ B200VIS_API int32_t b200vis_set_views(b200vis_ctx *ctx, uint32_t n_views, const 
  * GlobalTransform translation and ViewVisibility are read on the device), in query order. */
 B200VIS_API int32_t b200vis_set_lights(b200vis_ctx *ctx, uint32_t n_lights, const uint32_t *light_row, const float *range,
                            const uint64_t *layer_mask /* nullable */);
+/* The other objects assign_objects_to_clusters gathers (assign.rs:231-295), in its push order after the point lights: rect
+ * lights, then light probes (reflection probes and irradiance volumes interleaved in query order), then clustered decals.
+ * Each is clustered with the point-light walk (assign.rs:740-800) on a sphere centred at its GlobalTransform translation;
+ * only objects whose ViewVisibility is set this frame take part.  Radius per kind: rect light = range[j] (RectLight::range),
+ * probe = GlobalTransform::radius_vec3a(Vec3A::ONE), decal = GlobalTransform::scale().length() -- the last two are
+ * computed on the device from this frame's GlobalTransform (global_transform.rs:240-254).  Rect lights carry their own
+ * RenderLayers (layer_mask[j], first block; NULL = default layer); probes and decals the default layer.
+ *   Object j gets cluster ordinal n_lights + j (n_lights = the current b200vis_set_lights count): that is what
+ *   b200vis_download_clusters, b200vis_download_frame, the result sink and the bindings index map see, and b200vis_set_lights
+ *   shifts the ordinals of the objects when its count changes.  n_lights + n must be <= max_lights (B200VIS_ERR_CAPACITY).
+ *   kind[j] must be grouped in push order: 2 < {3, 4} < 5 (INVALID_ARG otherwise, as for a kind outside 2..5 or a row >=
+ *   max_entities); kind 1 (spot light) is B200VIS_ERR_UNSUPPORTED.  n = 0 removes the objects.
+ *   Refused: world_size > 1 (UNSUPPORTED: rank-major ordinals would break the grouping by kind), and UNIFORM cluster
+ *   bindings (INVALID_ARG, both ways round: the reference clusters none of these kinds without storage buffers).
+ * b200vis_set_shadow_lights ordinals still address the point lights only. */
+#define B200VIS_CLUSTERABLE_RECT_LIGHT        2u   /* = ClusterableObjectType::ordering().0 (assign.rs:115-131) */
+#define B200VIS_CLUSTERABLE_REFLECTION_PROBE  3u
+#define B200VIS_CLUSTERABLE_IRRADIANCE_VOLUME 4u
+#define B200VIS_CLUSTERABLE_DECAL             5u   /* 1 (spot light) is reserved: B200VIS_ERR_UNSUPPORTED */
+B200VIS_API int32_t b200vis_set_clusterable_objects(b200vis_ctx *ctx, uint32_t n, const uint32_t *kind, const uint32_t *row,
+                                                    const float *range /* rect lights; ignored otherwise; nullable if none */,
+                                                    const uint64_t *layer_mask /* rect lights; nullable => 1 */);
 B200VIS_API int32_t b200vis_set_cluster_view(b200vis_ctx *ctx, uint32_t view, const b200vis_cluster_view *params);
 /* Cluster grid dimensions of the view as last set (b200vis_set_cluster_view / b200vis_update_camera / b200vis_step);
  * zeros when clustering is off for the view.  The shim sizes Clusters::clusterable_objects from it. */
@@ -315,7 +338,7 @@ B200VIS_API int32_t b200vis_download_visible(b200vis_ctx *ctx, uint32_t view, ui
 B200VIS_API int32_t b200vis_download_visible_classes(b200vis_ctx *ctx, uint32_t view, uint8_t *classes, uint32_t capacity,
                                                      uint32_t *count);
 /* Clusters of one view in CSR form: offsets[n_clusters+1], light ordinals (index into the
- * b200vis_set_lights arrays; with world_size>1: global ordinal = rank-major) in the reference's
+ * b200vis_set_lights arrays, then the b200vis_set_clusterable_objects objects; with world_size>1: global ordinal = rank-major) in the reference's
  * push order, cluster index = (y*dims.x + x)*dims.z + z (assign.rs:676-678). */
 B200VIS_API int32_t b200vis_download_clusters(b200vis_ctx *ctx, uint32_t view, uint32_t *offsets, uint32_t *indices,
                                   uint32_t indices_capacity, uint32_t *total);
@@ -477,7 +500,12 @@ B200VIS_API int32_t b200vis_download_inherited_visibility(b200vis_ctx *ctx, uint
  *   UNIFORM  offsets_and_counts[4096] = pack_offset_and_counts (:855-859); index_lists[4096] = 16384 8-bit slots,
  *            truncated at ViewClusterBindings::MAX_INDICES exactly like the reference's record loop (:505-514)
  * gpu_index_of_light[n_map] = GlobalClusterableObjectMeta::entity_to_index for each light ordinal (NULL = the ordinal
- * itself); ordinals without an entry get the dummy index !0 (:703-705). */
+ * itself); ordinals without an entry get the dummy index !0 (:703-705).
+ * With clusterable objects set (STORAGE only), each cluster's counts are split by kind (ObjectsInClusterCpu::add_*,
+ * bevy_light/src/cluster/mod.rs:478-512).  Two limits of the bindings, not of Clusters: the index map is one per ordinal and
+ * shared by all views (the render world's per-view probe indices are not modelled), and an entity that is both an
+ * EnvironmentMapLight probe and an IrradianceVolume is one ordinal here where extract_clusters emits two records
+ * (bevy_pbr/src/cluster/mod.rs:454-463). */
 #define B200VIS_BINDINGS_OFF 0u
 #define B200VIS_BINDINGS_STORAGE 1u
 #define B200VIS_BINDINGS_UNIFORM 2u

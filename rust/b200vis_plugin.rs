@@ -22,7 +22,7 @@ use bevy::camera::primitives::{Aabb, Frustum, Sphere};
 use bevy::camera::visibility::*;
 use bevy::ecs::entity::EntityHashMap;
 use bevy::ecs::schedule::ScheduleCleanupPolicy::RemoveSystemsOnly;
-use bevy::light::{cluster::*, PointLight, SimulationLightSystems};
+use bevy::light::{cluster::*, EnvironmentMapLight, LightProbe, PointLight, RectLight, SimulationLightSystems};
 use bevy::prelude::*;
 use bevy::transform::{systems::*, TransformSystems};
 use core::any::TypeId;
@@ -68,6 +68,8 @@ extern "C" {
     fn b200vis_set_views(ctx: *mut b200vis_ctx, n: u32, views: *const b200vis_view) -> i32;
     fn b200vis_set_lights(ctx: *mut b200vis_ctx, n: u32, light_row: *const u32, range: *const f32, layers: *const u64) -> i32;
     fn b200vis_set_cluster_view(ctx: *mut b200vis_ctx, view: u32, p: *const b200vis_cluster_view) -> i32;
+    fn b200vis_set_clusterable_objects(ctx: *mut b200vis_ctx, n: u32, kind: *const u32, row: *const u32, range: *const f32,
+                                       layers: *const u64) -> i32;
     fn b200vis_host_cluster_view_setup(cfg: *const b200vis_cluster_config, camera_gt12: *const f32, clip_from_view16: *const f32,
                                        frustum: *const [f32; 4], layer_mask: u64, feedback: *const b200vis_cluster_feedback,
                                        planes_scratch: *mut f32, out: *mut b200vis_cluster_view) -> i32;
@@ -83,6 +85,8 @@ const F_INHERITED: u8 = 0x01; const F_AABB: u8 = 0x02; const F_SPHERE: u8 = 0x04
 const F_RANGE: u8 = 0x10; const F_SPHERE_FROM_GT: u8 = 0x40;
 const VIEW_ACTIVE: u8 = 1; const VIEW_NO_CPU_CULLING: u8 = 2;
 const ERR_HIERARCHY_CYCLE: i32 = 4;
+// ClusterableObjectType::ordering().0 (assign.rs:115-131) = B200VIS_CLUSTERABLE_*
+const KIND_RECT_LIGHT: u32 = 2; const KIND_REFLECTION_PROBE: u32 = 3; const KIND_IRRADIANCE_VOLUME: u32 = 4; const KIND_DECAL: u32 = 5;
 const MAX_VIEWS: usize = 8; const MAX_CLUSTERS: usize = 4096;
 
 /// Device context, the entity <-> row map, and the pinned host buffers the GPU writes into.  `Send + Sync`: exactly one
@@ -100,7 +104,8 @@ pub struct B200Vis {
     lights_epoch: u64,
     classes: Vec<TypeId>,         // VisibilityClass registry: bit k of the class mask = classes[k] (at most 8)
     view_entities: Vec<Entity>,   // view v of the device = this camera entity (query order of the cull system)
-    light_entities: Vec<Entity>,  // light ordinal -> entity (query order of the cluster system)
+    light_entities: Vec<Entity>,  // cluster ordinal -> entity: the point lights in query order, then the clusterable objects
+    object_kinds: Vec<u32>,       // kind of ordinal light_entities.len() - object_kinds.len() + j
     // sinks
     stats: Box<b200vis_frame_stats>,
     gt_col: Vec<[f32; 16]>, gt_bits: Vec<u32>, vv_col: Vec<u8>, vv_bits: Vec<u32>,
@@ -140,7 +145,7 @@ impl Plugin for B200VisibilityPlugin {
         let cluster_cap = 1usize << 18;
         let mut vis = B200Vis {
             ctx, max_entities: n, n: 0, row_of: Default::default(), entity_of: Vec::new(), columns_epoch: 0, bounds_epoch: u64::MAX,
-            lights_epoch: u64::MAX, classes: Vec::new(), view_entities: Vec::new(), light_entities: Vec::new(),
+            lights_epoch: u64::MAX, classes: Vec::new(), view_entities: Vec::new(), light_entities: Vec::new(), object_kinds: Vec::new(),
             stats: Box::default(), gt_col: vec![[0.0; 16]; n], gt_bits: vec![0; n.div_ceil(32)], vv_col: vec![0; n],
             vv_bits: vec![0; n.div_ceil(32)], visible_rows: vec![0; MAX_VIEWS * n], visible_classes: vec![0; MAX_VIEWS * n],
             cluster_offsets: vec![0; MAX_VIEWS * (MAX_CLUSTERS + 1)], cluster_indices: vec![0; MAX_VIEWS * cluster_cap], cluster_cap,
@@ -371,18 +376,29 @@ fn b200_check_visibility(
     Ok(())
 }
 
-/// cluster: the queries of assign_objects_to_clusters for point lights (assign.rs:137-153).
+/// cluster: the queries of assign_objects_to_clusters (assign.rs:137-178) except spot lights -- an app with spot lights keeps
+/// the reference system (INTEGRATION.md).
 fn b200_assign_lights_to_clusters(
     mut vis: ResMut<B200Vis>,
     mut views: Query<(Entity, &GlobalTransform, &Camera, &Frustum, Option<&ClusterConfig>, &mut Clusters, Option<&RenderLayers>)>,
     point_lights_query: Query<(Entity, &GlobalTransform, &ViewVisibility, Ref<PointLight>, Option<Ref<RenderLayers>>)>,
+    rect_lights_query: Query<(Entity, &GlobalTransform, &ViewVisibility, Ref<RectLight>, Option<Ref<RenderLayers>>)>,
+    light_probes_query: Query<(Entity, &GlobalTransform, &ViewVisibility, Has<EnvironmentMapLight>), With<LightProbe>>,
+    decals_query: Query<(Entity, &GlobalTransform, &ViewVisibility), With<ClusteredDecal>>,
     mut removed_lights: RemovedComponents<PointLight>,
+    mut removed_rect_lights: RemovedComponents<RectLight>,
+    mut removed_probes: RemovedComponents<LightProbe>,
+    mut removed_decals: RemovedComponents<ClusteredDecal>,
+    added_objects: Query<(), Or<(Added<LightProbe>, Added<ClusteredDecal>, Changed<EnvironmentMapLight>)>>,
     settings: Res<GlobalClusterSettings>,
 ) -> Result<(), BevyError> {
     let vis = &mut *vis;
     // ---- lights: ordinal = query order; positions and ViewVisibility are read on the device from the lights' own rows ----
-    let lights_changed = vis.lights_epoch != vis.columns_epoch || removed_lights.read().next().is_some()
-        || point_lights_query.iter().any(|(_, _, _, l, r)| l.is_changed() || r.is_some_and(|r| r.is_changed()));
+    let mut removed = removed_lights.read().count() + removed_rect_lights.read().count();
+    removed += removed_probes.read().count() + removed_decals.read().count();
+    let lights_changed = vis.lights_epoch != vis.columns_epoch || removed > 0 || !added_objects.is_empty()
+        || point_lights_query.iter().any(|(_, _, _, l, r)| l.is_changed() || r.is_some_and(|r| r.is_changed()))
+        || rect_lights_query.iter().any(|(_, _, _, l, r)| l.is_changed() || r.is_some_and(|r| r.is_changed()));
     if lights_changed {
         vis.light_entities.clear();
         let (mut rows, mut ranges, mut layers) = (Vec::new(), Vec::new(), Vec::new());
@@ -391,6 +407,25 @@ fn b200_assign_lights_to_clusters(
             vis.light_entities.push(e); rows.push(r); ranges.push(light.range); layers.push(layer.map_or(1, |l| l.bits()[0]));
         }
         vis.check(unsafe { b200vis_set_lights(vis.ctx, rows.len() as u32, rows.as_ptr(), ranges.as_ptr(), layers.as_ptr()) })?;
+        // the other kinds, in the reference's push order and under its settings gates (assign.rs:231-295); their radius and
+        // ViewVisibility are taken on the device from this frame's rows, only a rect light's range and layers are uploaded
+        let (mut kinds, mut orows, mut oranges, mut olayers) = (Vec::new(), Vec::new(), Vec::new(), Vec::new());
+        let mut push = |vis: &mut B200Vis, e: Entity, kind: u32, range: f32, layer: u64| {
+            let Some(&r) = vis.row_of.get(&e) else { return };
+            vis.light_entities.push(e); kinds.push(kind); orows.push(r); oranges.push(range); olayers.push(layer);
+        };
+        if settings.supports_storage_buffers {
+            for (e, _, _, light, layer) in rect_lights_query.iter() { push(vis, e, KIND_RECT_LIGHT, light.range, layer.map_or(1, |l| l.bits()[0])); }
+            for (e, _, _, is_reflection_probe) in light_probes_query.iter() {
+                push(vis, e, if is_reflection_probe { KIND_REFLECTION_PROBE } else { KIND_IRRADIANCE_VOLUME }, 0.0, 1);
+            }
+        }
+        if settings.clustered_decals_are_usable {
+            for (e, _, _) in decals_query.iter() { push(vis, e, KIND_DECAL, 0.0, 1); }
+        }
+        vis.check(unsafe { b200vis_set_clusterable_objects(vis.ctx, kinds.len() as u32, kinds.as_ptr(), orows.as_ptr(), oranges.as_ptr(),
+                                                           olayers.as_ptr()) })?;
+        vis.object_kinds = kinds;
         vis.lights_epoch = vis.columns_epoch;
     }
     // ---- per view: the prologue of assign_objects_to_clusters (assign.rs:324-485) through the library's host helper, which
@@ -443,8 +478,19 @@ fn b200_assign_lights_to_clusters(
         let mut cells = vec![ObjectsInClusterCpu::default(); nc];
         let off = &vis.cluster_offsets[v * (MAX_CLUSTERS + 1)..][..nc + 1];
         let idx = &vis.cluster_indices[v * vis.cluster_cap..];
+        let first_object = vis.light_entities.len() - vis.object_kinds.len();
         for (c, cell) in cells.iter_mut().enumerate() {
-            for i in off[c]..off[c + 1] { cell.add_point_light(vis.light_entities[idx[i as usize] as usize]); }   // ascending light order = push order (assign.rs:487)
+            for i in off[c]..off[c + 1] {                        // ascending ordinal = push order (assign.rs:487, 740-800)
+                let o = idx[i as usize] as usize;
+                let e = vis.light_entities[o];
+                if o < first_object { cell.add_point_light(e); continue; }
+                match vis.object_kinds[o - first_object] {
+                    KIND_RECT_LIGHT => cell.add_rect_light(e),
+                    KIND_REFLECTION_PROBE => cell.add_reflection_probe(e),
+                    KIND_IRRADIANCE_VOLUME => cell.add_irradiance_volume(e),
+                    _ => cell.add_decal(e),
+                }
+            }
         }
         clusters.clusterable_objects = ClusterableObjects::Cpu(cells);
         clusters.last_frame_total_cluster_index_count = Some(vis.stats.cluster_index_count[v] as usize);
